@@ -2,6 +2,7 @@
 """bench.py — throughput of the batched hot paths on N B200s (one process per GPU).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ekf|pf|mpc]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -19,10 +20,15 @@ index-addressed generators; the only inter-GPU traffic is one all-gather of 8 do
 libcrb's own NCCL communicator (crb_gather_stats) INSIDE the captured graph.
 
 Timing rules followed: W >= 3 warm-up steps; inputs rotate over 3 buffer sets whose total exceeds the
-126 MB L2; the K steps (+ stats tail + all-gather) are captured once and replayed >= 10 times, every replay
-timed with CUDA events on the launching stream, the whole series bracketed by barrier + synchronize, each replay's
-time maxed over ranks; `ms_per_step` is the MEDIAN replay / K and the minimum is reported beside it; SM clocks
-sampled with nvidia-smi during the timed region.
+126 MB L2; the K steps (+ stats tail + all-gather) are captured once in a CUDA graph, replayed once untimed, then
+once as the timed window: exactly K timed steps between two CUDA events on the launching stream, bracketed by
+barrier + synchronize, the window's time maxed over ranks; `ms_per_step` is the window / K; SM clocks sampled with
+nvidia-smi during the timed region.
+
+--dump-outputs DIR writes, after the timed steps, what the headline's last timed step returned to its caller
+(rank 0's shard): DIR/ekf_x.npy, the filtered states of all 2^20 agents, and DIR/ekf_P.npy, the covariances of a
+fixed seeded sample of 2^17 agents (DIR/ekf_P_agents.npy holds their indices), float32 (the indices float64),
+25 MB in all.  Inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the CPU restatement of the reference (oracle/, the only implementation of the
 path that can run here: Eigen/IPOPT are absent) on the box's host cores with all threads.
@@ -41,6 +47,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is compiled or cached in it at run time
 
 EKF_N = 1 << 20
 PF_N = int(os.environ.get("CRB_BENCH_PF_N", 1 << 20))     # diagnostics only: the contract workload is 2^20 x 8
@@ -285,18 +292,17 @@ def pinned(a):
 # =========================================================================================================
 # workloads: each returns a dict with value / ms_per_step / roofline / e2e / cpu_baseline pieces
 # =========================================================================================================
-REPLAYS = 10
 LAST_TIMING = {}
 
 
-def time_device_steps(step_fn, steps, warmup, world, after_fn=None, eng=None, graph=True, reps=None):
+def time_device_steps(step_fn, steps, warmup, world, after_fn=None, eng=None, graph=True):
     """W untimed steps, then the K steps (+ the optional tail: stats reduction and the all-gather) captured ONCE
-    into a CUDA graph and replayed `reps` (>= 10) times.  Every replay is timed with its own pair of CUDA events
-    on the launching stream; the series is bracketed by barrier + synchronize on both sides and each replay's time
-    is maxed over ranks.  Returns (median replay ms, mode); LAST_TIMING holds min / median / all replays.  If
-    capture is not possible the K steps are enqueued directly, also `reps` times."""
+    into a CUDA graph.  After barrier + synchronize the graph is replayed once untimed (upload and first-launch
+    costs) and, enqueued right behind it, once more as the timed window: exactly K timed steps between a pair of
+    CUDA events on the launching stream, then barrier + synchronize, the window's time maxed over ranks.  Returns
+    (window ms, mode); LAST_TIMING holds the record.  If capture is not possible the K steps are enqueued directly,
+    once, timed."""
     import torch
-    reps = REPLAYS if reps is None else reps
     for k in range(warmup):
         step_fn(k)
     if after_fn is not None:
@@ -314,43 +320,34 @@ def time_device_steps(step_fn, steps, warmup, world, after_fn=None, eng=None, gr
                 if after_fn is not None:
                     after_fn()
             eng.bind_current_stream()
-            g.replay()                      # one untimed replay
             mode = "cuda_graph"
         except Exception as exc:            # pragma: no cover - depends on driver / torch
             sys.stderr.write(f"graph capture failed ({exc}); timing direct launches\n")
             eng.bind_current_stream()
             g = None
     barrier_sync(world)
-    evs = []
-    for r in range(reps):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        if g is not None:
-            g.replay()
-        else:
-            for k in range(steps):
-                step_fn(warmup + k)
-            if after_fn is not None:
-                after_fn()
-        e1.record()
-        evs.append((e0, e1))
+    if g is not None:
+        g.replay()      # untimed; the GPU is still running it when e0 is reached, so no launch latency is timed
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    if g is not None:
+        g.replay()
+    else:
+        for k in range(steps):
+            step_fn(warmup + k)
+        if after_fn is not None:
+            after_fn()
+    e1.record()
     barrier_sync(world)
-    ms = torch.tensor([a.elapsed_time(b) for a, b in evs], dtype=torch.float64, device="cuda")
-    if world > 1:
-        import torch.distributed as dist
-        dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-    v = ms.cpu().numpy()
+    ms = max_over_ranks(e0.elapsed_time(e1), world)
     LAST_TIMING.clear()
-    LAST_TIMING.update(replays=int(reps), steps_per_replay=int(steps), ms_median=float(np.median(v)),
-                       ms_min=float(v.min()), ms_max=float(v.max()), mode=mode)
-    return float(np.median(v)), mode
+    LAST_TIMING.update(timed_steps=int(steps), ms=ms, mode=mode)
+    return ms, mode
 
 
 def timing_record(steps):
     t = dict(LAST_TIMING)
-    return dict(replays=t.get("replays"), steps_per_replay=t.get("steps_per_replay"),
-                ms_per_step_median=t.get("ms_median", 0.0) / steps, ms_per_step_min=t.get("ms_min", 0.0) / steps,
-                ms_per_step_max=t.get("ms_max", 0.0) / steps, launch=t.get("mode"))
+    return dict(timed_steps=t.get("timed_steps"), ms_per_step=t.get("ms", 0.0) / steps, launch=t.get("mode"))
 
 
 def time_host_steps(step_fn, steps, warmup, world):
@@ -476,7 +473,19 @@ def as_shipped_O0(fn, units, budget_s=1.0):
     return v
 
 
-def bench_ekf(eng, rank, world, steps, warmup, with_cpu):
+def dump_ekf(out_dir, x, P):
+    """The state of every agent and the covariance of a fixed seeded sample of 2^17 agents (P of all 2^20 would be
+    64 MB on its own)."""
+    import torch
+    agents = np.sort(np.random.default_rng(20).choice(x.shape[1], 1 << 17, replace=False))
+    idx = torch.from_numpy(agents).to(P.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("ekf_x", x.cpu().numpy()), ("ekf_P", P.index_select(1, idx).cpu().numpy()),
+                    ("ekf_P_agents", agents.astype(np.float64))):
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
+def bench_ekf(eng, rank, world, steps, warmup, with_cpu, dump_dir=None):
     import torch
     from cpprobotics_b200 import synth
     n = EKF_N
@@ -498,6 +507,8 @@ def bench_ekf(eng, rank, world, steps, warmup, with_cpu):
 
     ms, mode = time_device_steps(step, steps, warmup, world, after, eng=eng)
     timing = timing_record(steps)
+    if dump_dir is not None and rank == 0:
+        dump_ekf(dump_dir, *sets[(warmup + steps - 1) % NSETS][:2])    # step() updates x, P in place
     launches = steps + 2 + (1 if world > 1 else 0)   # K filter kernels + two stats-reduction kernels (+ NCCL's)
     value = world * n * steps / (ms * 1e-3)
     # roofline of the dominant kernel (one launch per step): algorithmic bytes / avg launch duration,
@@ -538,8 +549,7 @@ def bench_ekf(eng, rank, world, steps, warmup, with_cpu):
                              frac=achieved / peak, traffic=traffic_for("ekf"), peak_source=peak_src,
                              kernel="crb_ekf_step_kernel",
                              algorithmic_bytes_per_launch=EKF_BYTES * n,
-                             ms_per_launch_median=k_timing["ms_per_step_median"],
-                             ms_per_launch_min=k_timing["ms_per_step_min"],
+                             ms_per_launch=k_timing["ms_per_step"],
                              copy_gbs_same_run=copy_gbs, frac_of_copy_same_run=achieved / copy_gbs),
                e2e=dict(value=world * n * e_steps / (ms_e * 1e-3), unit="updates/s",
                         h2d_bytes_per_step=96 * n, d2h_bytes_per_step=80 * n,
@@ -758,8 +768,7 @@ def bench_mpc(eng, rank, world, steps, warmup, with_cpu, n=None, label=None, wit
                              frac=tfl / fpk, traffic=traffic, peak_source=fpk_src,
                              kernel=kernel, flop_model="executed iterations x (T-1) x (470 + 1.2 x 150) flop, DESIGN.md",
                              solves_per_s_kernel_only=world * n * steps / (ms_k * 1e-3),
-                             ms_per_launch_median=k_timing["ms_per_step_median"],
-                             ms_per_launch_min=k_timing["ms_per_step_min"],
+                             ms_per_launch=k_timing["ms_per_step"],
                              algorithmic_bytes_per_launch=MPC_BYTES * n,
                              traffic_over_algorithmic=(traffic / (MPC_BYTES * n)) if traffic else None,
                              io_gbs=achieved_io, io_frac_of_hbm=achieved_io / peak))
@@ -781,10 +790,8 @@ def bench_mpc(eng, rank, world, steps, warmup, with_cpu, n=None, label=None, wit
                 eng.stats_reduce(cost, status, iters2, i0=rank * n, out=stats)
                 gather_stats(stats, world, eng, out=table)
             ms_h, _ = time_device_steps(step_hinted, steps, 1, world, eng=eng)
-            t_h = timing_record(steps)
             same = bool(torch.equal(iters2, want_iters)) and bool(torch.equal(cost, want_cost))
             hinted[name] = dict(value=world * n * steps / (ms_h * 1e-3), unit="solves/s", ms_per_step=ms_h / steps,
-                                ms_per_step_median=t_h["ms_per_step_median"], ms_per_step_min=t_h["ms_per_step_min"],
                                 speedup_vs_index_order=ms / ms_h, same_bits_as_index_order=same)
         hinted["what"] = ("crb_mpc_solve_batched_hinted: iteration counts of the agents' previous solve as scheduling "
                           "hints (receding-horizon MPC), stats + gather included like the headline step; "
@@ -1042,7 +1049,7 @@ def run_ours(args):
     if cpu:
         restore, pin_note = cpu_pin_one_numa_node()
     with ClockSampler(local) as clk:
-        head = bench_ekf(eng, rank, world, args.steps, args.warmup, with_cpu=cpu)
+        head = bench_ekf(eng, rank, world, args.steps, args.warmup, with_cpu=cpu, dump_dir=args.dump_outputs)
         if args.workload in ("all", "pf"):
             res["pf"] = bench_pf(eng, rank, world, args.steps, args.warmup, with_cpu=cpu)
         if args.workload in ("all", "pf"):
@@ -1183,6 +1190,8 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="all", choices=["all", "ekf", "ekf100", "ekf16m", "pf", "mpc", "lqr"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's last timed step's outputs to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":

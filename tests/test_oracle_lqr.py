@@ -1,6 +1,5 @@
 """CPU: solve_DARE()/dlqr() restatement (row f-4) against SciPy's DARE solution, the reference's own text
 (oracle/_ref) and its iteration semantics."""
-import ctypes as C
 import os
 
 import numpy as np
@@ -10,8 +9,7 @@ import scipy.linalg as sl
 from cpprobotics_b200 import synth
 from oracle import oracle as O
 
-REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
-f32p = np.ctypeslib.ndpointer(np.float32, flags="C_CONTIGUOUS")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_text_golden.npz")
 
 
 @pytest.mark.parametrize("nx,nu", [(4, 1), (5, 2)])
@@ -41,19 +39,11 @@ def test_iteration_cap_and_tolerance_semantics():
 
 @pytest.mark.parametrize("nx,nu,lib", [(4, 1, "libref_lqr4.so"), (5, 2, "libref_lqr5.so")])
 def test_restatement_is_bitwise_the_reference_text(nx, nu, lib):
-    path = os.path.join(REF, lib)
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref not built")
-    L = C.CDLL(path)
-    A, B, Q, R = synth.lqr_inputs(200, nx, seed=12)
+    """K and X of the reference's solve_DARE/dlqr (`lib`, the reference source compiled through the shims) on
+    200 seeded systems, as stored by tests/golden/make_ref_text_golden.py."""
+    G = np.load(GOLDEN)
+    A, B, Q, R = (G[f"lqr{nx}_{k}"] for k in "ABQR")
     r = O.dlqr_batched(A, B, Q, R, nx, nu)
     for i in range(200):
-        K, X = np.zeros(nu * nx, np.float32), np.zeros(nx * nx, np.float32)
-        a, b = np.ascontiguousarray(A[:, i]), np.ascontiguousarray(B[:, i])
-        if nx == 4:
-            L.ref_dlqr4.argtypes = [f32p, f32p, f32p, C.c_float, f32p, f32p]
-            L.ref_dlqr4(a, b, Q, float(R[0]), K, X)
-        else:
-            L.ref_dlqr5.argtypes = [f32p] * 6
-            L.ref_dlqr5(a, b, Q, R, K, X)
+        K, X = G[f"lqr{nx}_K"][:, i], G[f"lqr{nx}_X"][:, i]
         assert np.array_equal(K, r["K"][:, i]) and np.array_equal(X, r["X"][:, i])

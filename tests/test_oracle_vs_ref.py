@@ -1,80 +1,54 @@
 """CPU: pins the oracle against the reference's OWN source files, compiled unmodified against header shims
 (oracle/shim -> oracle/_ref/libref_*.so; see oracle/shim/README.md for what this does and does not pin).
-Skipped when oracle/_ref was not built (it is built whenever /root/reference is present)."""
-import ctypes as C
+What those files returned is stored in tests/golden/ref_text_golden.npz (tests/golden/make_ref_text_golden.py
+regenerates it where the reference tree is present), so the pin holds in every checkout."""
 import os
 
 import numpy as np
-import pytest
 
 import ref_mpc as M
 from cpprobotics_b200 import synth
 from oracle import oracle as O
 
-REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
-f32p = np.ctypeslib.ndpointer(np.float32, flags="C_CONTIGUOUS")
-f64p = np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS")
-
-
-def _load(name):
-    path = os.path.join(REF, name)
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref not built (needs /root/reference: make -C oracle ref)")
-    return C.CDLL(path)
+G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_text_golden.npz"))
 
 
 def test_ekf_restatement_is_bitwise_the_reference_text():
-    L = _load("libref_ekf.so")
-    L.ref_motion_model.argtypes = [f32p, f32p, f32p]
-    L.ref_jacobF.argtypes = [f32p, f32p, f32p]
-    L.ref_ekf_estimation.argtypes = [f32p] * 6
     n = 3000
     x, P, z, u = synth.ekf_inputs(n, seed=31)
     dt, Q, R = O.ekf_constants()
     lib = O.lib()
     for i in range(n):
         xi, ui = np.ascontiguousarray(x[:, i]), np.ascontiguousarray(u[:, i])
-        a, b = np.zeros(4, np.float32), np.zeros(4, np.float32)
-        L.ref_motion_model(xi, ui, a); lib.crb_oracle_motion_model(xi, ui, dt, b)
-        assert np.array_equal(a, b)
-        ja, jb = np.zeros(16, np.float32), np.zeros(16, np.float32)
-        L.ref_jacobF(xi, ui, ja); lib.crb_oracle_jacobF(xi, ui, dt, jb)
-        assert np.array_equal(ja, jb)
-        xr, Pr = xi.copy(), np.ascontiguousarray(P[:, i]).copy()
-        L.ref_ekf_estimation(xr, Pr, np.ascontiguousarray(z[:, i]), ui, Q, R)
+        b = np.zeros(4, np.float32)
+        lib.crb_oracle_motion_model(xi, ui, dt, b)
+        assert np.array_equal(G["ekf_motion"][:, i], b)
+        jb = np.zeros(16, np.float32)
+        lib.crb_oracle_jacobF(xi, ui, dt, jb)
+        assert np.array_equal(G["ekf_jacobF"][:, i], jb)
         xo, Po = O.ekf_estimation(xi, P[:, i], z[:, i], ui)
-        assert np.array_equal(xr, xo) and np.array_equal(Pr, Po)
+        assert np.array_equal(G["ekf_x_out"][:, i], xo) and np.array_equal(G["ekf_P_out"][:, i], Po)
 
 
 def test_ekf_known_answer_through_the_reference_text():
-    L = _load("libref_ekf.so")
-    L.ref_ekf_estimation.argtypes = [f32p] * 6
-    dt, Q, R = O.ekf_constants()
-    x, P = np.zeros(4, np.float32), np.eye(4, dtype=np.float32).reshape(-1).copy()
-    L.ref_ekf_estimation(x, P, np.float32([0.1, 0.0]), np.float32([1.0, 0.1]), Q, R)
+    x, P = G["ekf_ka_x"], G["ekf_ka_P"]
     np.testing.assert_allclose(x, [0.1, 0.0, 0.010000001, 1.0], atol=1e-8)
     assert abs(P[0] - 0.50495052) < 1e-7 and abs(P[15] - 1.0050495) < 1e-7
+    xo, Po = O.ekf_estimation(np.zeros(4, np.float32), np.eye(4, dtype=np.float32).reshape(-1),
+                              np.float32([0.1, 0.0]), np.float32([1.0, 0.1]))
+    assert np.array_equal(x, xo) and np.array_equal(P, Po)
 
 
 def test_pf_restatement_is_bitwise_the_reference_text():
-    L = _load("libref_pf.so")
-    L.ref_gauss_likelihood.restype = C.c_float
-    L.ref_gauss_likelihood.argtypes = [C.c_float, C.c_float]
-    L.ref_pf_np.restype = C.c_int
-    L.ref_pf_localization.argtypes = [f32p, f32p, f32p, f32p, f32p, C.c_int, f32p, f32p, C.c_float, C.c_uint, f64p]
-    for xv in np.linspace(-0.6, 0.6, 101):
+    for xv, ref in zip(np.linspace(-0.6, 0.6, 101), G["pf_gauss"]):
         s = float(np.sqrt(np.float32(0.01)))
-        assert L.ref_gauss_likelihood(xv, s) == np.float32(O.gauss_likelihood(xv, s))
-    NP = L.ref_pf_np()
+        assert ref == np.float32(O.gauss_likelihood(xv, s))
+    NP = int(G["pf_np"])
     assert NP == 100                                    # src/particle_filter.cpp:21
     px, pw, _ = synth.pf_inputs(NP, seed=9)
     lm = synth.pf_landmarks(4, seed=9)                  # the reference sees <= 4 landmarks (:192-196)
     c = O.pf_constants()
-    pxr = np.ascontiguousarray(px.T.reshape(-1)).copy() # 4xNP column-major == [NP][4]
-    pwr = pw.copy()
-    xe, Pe, draws = np.zeros(4, np.float32), np.zeros(16, np.float32), np.zeros(2 * NP)
-    L.ref_pf_localization(pxr, pwr, xe, Pe, np.ascontiguousarray(lm.reshape(-1)), len(lm), c["u"], c["rsim_diag"],
-                          float(c["Q"]), 4242, draws)
+    pxr, pwr, xe, Pe, draws = (G[k] for k in ("pf_px_out", "pf_pw_out", "pf_xEst", "pf_PEst", "pf_draws"))
     lib = O.lib()
     pxo, pwo = np.zeros((NP, 4), np.float32), np.zeros(NP, np.float32)
     for ip in range(NP):
@@ -82,7 +56,7 @@ def test_pf_restatement_is_bitwise_the_reference_text():
         lib.crb_oracle_pf_particle(xx, ww, np.ascontiguousarray(draws[2 * ip:2 * ip + 2]), c["u"], c["rsim_diag"],
                                    np.ascontiguousarray(lm.reshape(-1)), len(lm), float(c["Q"]), c["dt"], c["pi"])
         pxo[ip], pwo[ip] = xx, ww[0]
-    assert np.array_equal(pxr.reshape(NP, 4), pxo)      # predict: bit for bit
+    assert np.array_equal(pxr, pxo)                     # predict: bit for bit
     s = np.float32(0.0)
     for w in pwo:                                       # pw / pw.sum() with Eigen's float sum (:104)
         s = np.float32(s + w)
@@ -93,56 +67,38 @@ def test_pf_restatement_is_bitwise_the_reference_text():
 
 
 def test_mpc_helpers_are_bitwise_the_reference_text():
-    L = _load("libref_mpc.so")
-    L.ref_mpc_T.restype = C.c_int
-    L.ref_update.argtypes = [f32p, C.c_float, C.c_float]
-    L.ref_calc_nearest_index.restype = C.c_int
-    L.ref_calc_nearest_index.argtypes = [f32p, f32p, f32p, f32p, C.c_int, C.c_int]
-    L.ref_calc_ref_trajectory.argtypes = [f32p, f32p, f32p, f32p, f32p, C.c_int, C.c_float, C.POINTER(C.c_int), f32p]
-    T = L.ref_mpc_T()
+    T = int(G["mpc_T"])
     assert T == 6                                       # src/model_predictive_control.cpp:24
-    rng = np.random.default_rng(2)
-    for _ in range(500):                                # update(): :69-81
-        st = np.float32([rng.uniform(-50, 50), rng.uniform(-50, 50), rng.uniform(-3, 3), rng.uniform(-6, 15.4)])
-        a, d = np.float32(rng.uniform(-1.5, 1.5)), np.float32(rng.uniform(-1, 1))
-        r = st.copy(); L.ref_update(r, a, d)
+    for st, (a, d), r in zip(G["upd_state"], G["upd_ad"], G["upd_out"]):     # update(): :69-81
         assert np.array_equal(r, O.plant_update(st, a, d))
     course = synth.mpc_course()
     cx, cy, cyaw, sp = course
-    st, pind = synth.mpc_states(400, seed=3, course=course)
-    for i in range(400):
+    st, pind = G["crt_state"], G["crt_pind"]
+    for i in range(st.shape[1]):
         s = np.ascontiguousarray(st[:, i])
-        assert L.ref_calc_nearest_index(s, cx, cy, cyaw, len(cx), int(pind[i])) == O.calc_nearest_index(s, cx, cy, int(pind[i]))
-        ti = C.c_int(int(pind[i])); xr = np.zeros(4 * T, np.float32)
-        L.ref_calc_ref_trajectory(s, cx, cy, cyaw, sp, len(cx), 1.0, C.byref(ti), xr)
+        assert G["crt_nearest"][i] == O.calc_nearest_index(s, cx, cy, int(pind[i]))
         xo, to = O.calc_ref_trajectory(s, cx, cy, cyaw, sp, 1.0, T, int(pind[i]))
-        assert ti.value == to and np.array_equal(xr, xo.reshape(-1))
+        assert G["crt_tind"][i] == to and np.array_equal(G["crt_xref"][i], xo.reshape(-1))
 
 
 def test_nlp_statement_equals_fg_eval_and_solution_satisfies_it():
     """FG_EVAL::operator() (:199-252) evaluated by the reference's own code: (a) our statement of the cost
     (tests/ref_mpc.nlp_cost) is the same function, (b) the solver's answer is feasible for the reference's
     constraints and its reported cost is the reference's fg[0]."""
-    L = _load("libref_mpc.so")
-    L.ref_fg_eval.argtypes = [f32p, f64p, f64p]
     T = 6
-    course = synth.mpc_course()
-    st, pind = synth.mpc_states(40, seed=4, course=course)
-    xref, _ = synth.mpc_xref_numpy(st, pind, T, course=course)
+    st, xref = G["nlp_state"], G["nlp_xref"]
     r = O.mpc_solve_batched(st, xref, T)
-    rng = np.random.default_rng(0)
-    for i in range(40):
+    # the reference evaluated its constraints at this solution when the fixture was made
+    np.testing.assert_allclose(r["sol"], G["nlp_sol"], rtol=0, atol=1e-6)
+    for i in range(st.shape[1]):
         xr = np.ascontiguousarray(xref[:, i])           # field 4t+k == 4xT column-major
         # (a) random point: cost identity
-        v = rng.normal(size=4 * T + 2 * (T - 1))
-        fg = np.zeros(1 + 4 * T)
-        L.ref_fg_eval(xr, v, fg)
+        v, fg = G["nlp_vars"][i], G["nlp_fg_vars"][i]
         X = v[:4 * T].reshape(4, T); U = v[4 * T:].reshape(2, T - 1)
         p = dict(M.DEFAULTS)
         assert abs(fg[0] - M.nlp_cost(X, U, xr.reshape(T, 4).T.astype(float), p)) <= 1e-9 * abs(fg[0])
         # (b) the oracle's solution
-        sol = r["sol"][:, i].astype(np.float64)
-        L.ref_fg_eval(xr, sol, fg)
+        fg = G["nlp_fg_sol"][i]
         assert abs(fg[0] - r["cost"][i]) <= 2e-5 * max(1.0, fg[0])
         g = fg[1:].reshape(4, T)                        # rows x, y, yaw, v; column 0 = initial state
         assert np.array_equal(g[:, 0].astype(np.float32), st[:, i])
@@ -152,18 +108,8 @@ def test_nlp_statement_equals_fg_eval_and_solution_satisfies_it():
 def test_resampling_restatement_is_bitwise_the_reference_text():
     """resampling() + cumsum() (:111-148) of the reference's own source against oracle.pf_resample in
     reference_mode, on peaked weights (Neff < NP/2 -> resample) and on flat ones (no resample)."""
-    L = _load("libref_pf.so")
-    L.ref_resampling.restype = C.c_int
-    L.ref_resampling.argtypes = [f32p, f32p, C.c_uint, f64p]
-    NP = 100
     for seed, sharp in ((1, True), (2, True), (3, False)):
-        px, pw, noise = synth.pf_inputs(NP, seed=seed)
-        lm = synth.pf_landmarks(4, seed=seed)
-        if sharp:
-            px, pw = O.pf_predict_weight_batched(px, pw, noise, lm)
-            pw = (pw / np.float32(pw.sum())).astype(np.float32)
-        pxr, pwr, draws = np.ascontiguousarray(px.T.reshape(-1)).copy(), pw.copy(), np.zeros(NP)
-        did_r = L.ref_resampling(pxr, pwr, 99 + seed, draws)
+        px, pw, draws = G[f"rs{seed}_px"], G[f"rs{seed}_pw"], G[f"rs{seed}_draws"]
         pxo, pwo, did_o, neff = O.pf_resample(px, pw, draws, reference_mode=True)
-        assert bool(did_r) == did_o == sharp
-        assert np.array_equal(pxr.reshape(NP, 4).T, pxo) and np.array_equal(pwr, pwo)
+        assert bool(G[f"rs{seed}_did"]) == did_o == sharp
+        assert np.array_equal(G[f"rs{seed}_px_out"], pxo) and np.array_equal(G[f"rs{seed}_pw_out"], pwo)
